@@ -8,7 +8,13 @@ N>1: BASELINE config 4 -- one process per GPU (torchrun), 16 keyframes per GPU (
 the whole-model objects (`full_model*`) include the NCCL all-gather of the per-rank `result` maps in their timed region.
 `--config hires` is BASELINE config 5: 512x1024, 64 planes, 6 source frames, batch 4 per GPU.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config default|hires]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config default|hires] [--dump-outputs DIR]
+
+`--steps K` is the number of timed steps of the cost-volume path, on the device and through the host-buffer entry (e2e),
+or of the reference arm (default 200; 5 for the slow reference arm).  The informational whole-model, loss and CPU-baseline
+timings keep their own fixed counts.  `--dump-outputs DIR` writes what the last timed step computed (rank 0's cost volume and
+single-frame volumes; the oracle port's in the reference arm) to DIR/<name>.npy, sampled as dump_outputs() describes, so
+that two builds run with the same arguments can be compared.
 
 `--impl reference` times the reference's CPU implementation of the path.  The reference is pure Python/PyTorch and
 cannot travel to the GPU box, so this arm runs the oracle port (oracle/cost_volume_oracle.py: the same torch CPU
@@ -163,7 +169,7 @@ def cpu_port_keyframes_per_s(repeats, threads=None):
 def run_reference(args, rank):
     if rank != 0:
         return
-    steps = max(1, min(args.steps, 5))
+    steps = args.steps
     from oracle import cost_volume_oracle as O
     from monorec_b200.synthetic import make_inputs
     data = make_inputs(1, F, H, W, seed=0)
@@ -180,8 +186,10 @@ def run_reference(args, rank):
     torch.set_num_threads(min(trial, key=trial.get))
     t0 = time.perf_counter()
     for _ in range(steps):
-        O.cost_volume_torch(data, INV_HI, INV_LO, D)
+        cv, sf = O.cost_volume_torch(data, INV_HI, INV_LO, D)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, cv, torch.stack(sf))
     val = steps / dt
     line = {"impl": "reference", "metric": METRIC, "value": val, "unit": "keyframes/s", "n_gpus": args.gpus,
             "steps": steps, "warmup": 1 + len(candidates), "ms_per_step": 1e3 * dt / steps, "higher_is_better": True,
@@ -192,6 +200,25 @@ def run_reference(args, rank):
                              "sample": f"{steps} x 1 keyframe, torch CPU ops, {torch.get_num_threads()} threads (fastest of {candidates})"},
             "e2e": {"value": val, "unit": "keyframes/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}
     emit(line)
+
+
+DUMP_BYTES = 48 << 20                     # at most this much float32 in one --dump-outputs directory
+
+
+def dump_outputs(out_dir, cv, sfcv):
+    """Writes the cost-volume outputs as float32 .npy files: cost_volume.npy [N, D] and single_frame_cvs.npy [N, F, D],
+    the full depth-plane profile of N pixels (b, y, x).  The pixels are the first N of a permutation drawn from a CPU
+    generator with a fixed seed, in ascending order, N as large as DUMP_BYTES allows (every pixel if all fit): the same
+    arguments dump the same pixels on every run and every build."""
+    import numpy as np
+    nF, B, nD, h, w = sfcv.shape
+    n = min(B * h * w, DUMP_BYTES // (4 * nD * (1 + nF)))
+    pix = torch.randperm(B * h * w, generator=torch.Generator().manual_seed(0))[:n].sort().values.to(cv.device)
+    b, y, x = pix // (h * w), pix // w % h, pix % w
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    np.save(out_dir / "cost_volume.npy", cv[b, :, y, x].float().cpu().numpy())
+    np.save(out_dir / "single_frame_cvs.npy", sfcv.permute(1, 3, 4, 0, 2)[b, y, x].float().cpu().numpy())
 
 
 _REAL_STDOUT = None
@@ -219,14 +246,19 @@ def main():
     quiet_stdout()
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default 200; 5 with --impl reference)")
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", default="default", choices=["default", "hires"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-full-model", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps is None:
+        args.steps = 5 if args.impl == "reference" else 200
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -235,7 +267,6 @@ def main():
         run_reference(args, rank)
         return
     args.warmup = max(args.warmup, 3)      # timing rules: at least 3 warm-up steps (the JSON line reports the number used)
-    args.steps = max(args.steps, 1)
     assert torch.cuda.is_available(), "bench.py needs a GPU (no CPU fallback in the product path)"
     numa_cpus = pin_to_gpu_numa_node(local)
     torch.cuda.set_device(local)
@@ -297,6 +328,8 @@ def main():
         barrier()
     ms = ev0.elapsed_time(ev1)
     launches = _lib.launch_count(reset=True)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, cv, sfcv)
     t = torch.tensor([ms], device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -346,12 +379,11 @@ def main():
             _lib.check(lib.mr_cost_volume_host(h_key.data_ptr(), h_frames.data_ptr(), h_kp.data_ptr(), h_kk.data_ptr(),
                                                h_poses.data_ptr(), h_intr.data_ptr(), h_cv.data_ptr(), None,
                                                B, F, D, H, W, INV_LO, INV_HI, 10.0, ws.data_ptr(), ws_bytes), "e2e")
-        e_steps = max(3, min(args.steps, 10))
         for _ in range(3):
             e2e_step()
         barrier()
         t0 = time.perf_counter()
-        for _ in range(e_steps):
+        for _ in range(args.steps):
             e2e_step()      # synchronous: returns after the last D2H copy has landed
         torch.cuda.synchronize()
         dt = time.perf_counter() - t0
@@ -361,8 +393,8 @@ def main():
         if rank == 0:
             h2d = (1 + F) * B * 3 * H * W * 4 + (2 + 2 * F) * B * 64
             d2h = B * D * H * W * 4
-            line["e2e"] = {"value": world * B * e_steps / float(t.item()), "unit": "keyframes/s",
-                           "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h, "steps": e_steps,
+            line["e2e"] = {"value": world * B * args.steps / float(t.item()), "unit": "keyframes/s",
+                           "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h, "steps": args.steps,
                            "api": "mr_cost_volume_host (C ABI, pinned host buffers NUMA-local to the GPU; images and matrices "
                                   "uploaded, fused cost volume downloaded, single-frame volumes left on the device for the "
                                   "MaskModule as in monorec_model.py:693-699)"}

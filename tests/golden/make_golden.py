@@ -26,6 +26,9 @@ Files written
                           w.r.t. the predicted inverse depth on seeded inputs, three argument sets (`--only-reprojection`)
   model_fp64.npz          the same two model configurations evaluated by the reference in float64 (`--only-model-fp64`):
                           the reference's own fp32 rounding noise on `result` / `cv_mask`, which sizes the GPU gates
+  integration.json        the "models" block of configs/evaluate/eval_monorec.json, the reference MonoRecModel's constructor
+                          keywords, and the settings of the models the reference's ConfigParser builds from that block
+                          (`--only-integration`)
 """
 import os
 import sys
@@ -305,6 +308,29 @@ def main():
             print(tag, "inf share", float(inf.float().mean()), "mean finite error", float(err[~inf].mean()),
                   "max |grad|", float(pred.grad.abs().max()), "reduced", float(red))
         np.savez_compressed(HERE / "reprojection.npz", **out)
+        return
+    if "--only-integration" in sys.argv:
+        # INTEGRATION.md section 2 on the reference side: evaluate.py:29-31 builds its models with
+        # ConfigParser.initialize_list("models", model.model) from the config's "models" block.  The checkpoint path is
+        # dropped (no checkpoint offline); the parser is created without its run directories and logging set-up.
+        import inspect
+        import json
+        import model.model as module_arch  # noqa
+        from utils.parse_config import ConfigParser  # noqa
+        cfg = json.loads((REF / "configs" / "evaluate" / "eval_monorec.json").read_text())
+        models = [dict(m, args={k: v for k, v in m["args"].items() if k != "checkpoint_location"}) for m in cfg["models"]]
+        parser = ConfigParser.__new__(ConfigParser)
+        parser._config = {"models": models}
+        keywords = [n for n in inspect.signature(ref_mod.MonoRecModel.__init__).parameters if n != "self"]
+        settings = []
+        for m in parser.initialize_list("models", module_arch):
+            vals = {n: getattr(m, n) for n in keywords if hasattr(m, n)}
+            settings.append({n: (list(v) if isinstance(v, tuple) else v) for n, v in vals.items()
+                             if isinstance(v, (bool, int, float, str, list, tuple, type(None)))})
+        out = {"config": "configs/evaluate/eval_monorec.json", "models": models, "reference_init_keywords": keywords,
+               "reference_settings": settings}
+        (HERE / "integration.json").write_text(json.dumps(out, indent=1) + "\n")
+        print(json.dumps(settings))
         return
     if "--only-d64f6" in sys.argv:
         # BASELINE config 5's plane and frame counts (64 planes, 6 source frames) at a small size; added after the other

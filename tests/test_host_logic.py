@@ -1,6 +1,5 @@
 """Host-side logic that needs no GPU: checkpoint contract, padding arithmetic, descriptor ABI, weight packing."""
 import ctypes
-from pathlib import Path
 
 import pytest
 import torch
@@ -166,61 +165,29 @@ def test_c_subpixel_kernels_reproduce_reference_layers():
     assert torch.allclose(out, ref, atol=1e-5)
 
 
-def test_integration_monkey_patch_resolves_through_reference_config_parser():
-    """INTEGRATION.md section 2 executed against the unmodified reference (dev container only; the GPU box has no /root/reference):
-    after the two-line patch, the reference's own registry path -- utils/parse_config.ConfigParser.initialize("arch",
-    model.model) as evaluate.py:29-31 calls it, with the "arch" block of configs/evaluate/eval_monorec.json -- constructs the
-    drop-in, with the reference's constructor keywords."""
-    import importlib
+def test_integration_monkey_patch_resolves_through_reference_config_parser(golden_dir):
+    """INTEGRATION.md section 2: the reference builds its models by class name -- evaluate.py:29-31 calls
+    ConfigParser.initialize_list("models", model.model), which looks every entry's "type" up in model.model and calls it
+    with the entry's "args".  After the two-line patch that lookup yields the drop-in; fed the "models" block of
+    configs/evaluate/eval_monorec.json, it must build monorec_b200's model, accept the reference constructor's keywords in
+    the reference's order, and end up with the settings the reference's own model has (tests/golden/integration.json,
+    written by `make_golden.py --only-integration` from the unmodified reference)."""
+    import inspect
     import json
-    import os
-    import sys
     import types
-    ref = Path(os.environ.get("MONOREC_REFERENCE", "/root/reference"))
-    if not (ref / "utils" / "parse_config.py").is_file():
-        pytest.skip("reference tree not available")
-    for name in ["kornia", "kornia.augmentation", "kornia.geometry", "kornia.geometry.camera", "kornia.geometry.depth"]:
-        sys.modules.setdefault(name, types.ModuleType(name))          # SURVEY.md Appendix B shims (kornia is not installed)
-    sys.modules["kornia.augmentation"].RandomHorizontalFlip = object
-    sys.modules["kornia.augmentation"].RandomResizedCrop = object
-    sys.modules["kornia.geometry.camera"].pixel2cam = None
-    sys.modules["kornia.geometry.depth"].DepthWarper = None
-    sys.modules["kornia"].augmentation = sys.modules["kornia.augmentation"]
-    sys.path.insert(0, str(ref))
-    saved = {k: sys.modules.get(k) for k in ("model", "model.model", "model.monorec", "model.monorec.monorec_model", "utils", "utils.parse_config")}
-    try:
-        import monorec_b200.model as fast
-        ref_mod = importlib.import_module("model.monorec.monorec_model")
-        module_arch = importlib.import_module("model.model")
-        assert module_arch.MonoRecModel is ref_mod.MonoRecModel           # the stock registry
-        # ---- INTEGRATION.md, "without touching the reference tree" ----
-        ref_mod.MonoRecModel = fast.MonoRecModel
-        sys.modules["model.model"].MonoRecModel = fast.MonoRecModel
-        # ---- the reference's own resolution path ----
-        parse_config = importlib.import_module("utils.parse_config")
-        cfg = json.loads((ref / "configs" / "evaluate" / "eval_monorec.json").read_text())
-        parser = parse_config.ConfigParser.__new__(parse_config.ConfigParser)   # no run directories / logging set-up
-        entries = []
-        for m in cfg["models"]:                                                 # evaluate.py:29-31: initialize_list("models", ...)
-            m = dict(m)
-            m["args"] = {k: v for k, v in m["args"].items() if k != "checkpoint_location"}   # no checkpoint offline
-            entries.append(m)
-        parser._config = {"models": entries, "arch": entries[0]}
-        if not isinstance(getattr(parse_config.ConfigParser, "config", None), property):
-            parser.config = parser._config
-        built = list(parser.initialize_list("models", module_arch)) + [parser.initialize("arch", module_arch)]
-        for model in built:
-            assert type(model) is fast.MonoRecModel and type(model).__module__ == "monorec_b200.model"
-            assert model.use_mono is True and model.use_stereo is False and model.pretrain_mode == 0
-            assert tuple(model.inv_depth_min_max) == (0.33, 0.0025)
-    finally:
-        for k, v in saved.items():
-            if v is None:
-                sys.modules.pop(k, None)
-            else:
-                sys.modules[k] = v
-        if str(ref) in sys.path:
-            sys.path.remove(str(ref))
+    import monorec_b200.model as fast
+    g = json.loads((golden_dir / "integration.json").read_text())
+    assert [n for n in inspect.signature(fast.MonoRecModel.__init__).parameters if n != "self"] == g["reference_init_keywords"]
+    module_arch = types.ModuleType("model.model")          # the reference's model/model.py registry ...
+    module_arch.MonoRecModel = fast.MonoRecModel            # ... after INTEGRATION.md's patch
+    assert g["models"] and len(g["models"]) == len(g["reference_settings"])
+    for entry, ref in zip(g["models"], g["reference_settings"]):
+        model = getattr(module_arch, entry["type"])(**entry["args"])
+        assert type(model) is fast.MonoRecModel and type(model).__module__ == "monorec_b200.model"
+        got = {n: getattr(model, n) for n in ref}
+        assert {n: (list(v) if isinstance(v, tuple) else v) for n, v in got.items()} == ref
+        assert model.use_mono is True and model.use_stereo is False and model.pretrain_mode == 0
+        assert tuple(model.inv_depth_min_max) == (0.33, 0.0025)
 
 
 def test_trunk_unused_level_is_lazy_and_identical():
