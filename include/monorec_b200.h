@@ -128,7 +128,7 @@ int mr_cost_volume_host(const float* h_keyframe, const float* h_frames,
 #define MR_DT_F32 0
 #define MR_DT_F16 1           /* IEEE half storage: tensor-core path (kind::f16, fp32 accumulate) and the helper kernels */
 #define MR_ACT_NONE 0
-#define MR_ACT_LEAKY 1     /* x >= 0 ? x : act_a * x */
+#define MR_ACT_LEAKY 1     /* x >= 0 ? x : act_a * x  (any slope, on every path) */
 #define MR_ACT_SIGMOID 2
 #define MR_ACT_ABSTANH 3   /* act_a + act_b * |tanh(x)|  (depth heads + inverse-depth affine, monorec_model.py:717) */
 
@@ -169,6 +169,33 @@ int mr_conv2d_nhwc_tc(const mr_conv_desc* desc, int n_pad, int k_pad, int round_
  * (anything else: MR_EINVAL).  Tiles are ordered (spatial tile, phase), so the phases of a tile run side by side and the input is
  * read from HBM once instead of once per phase.  n_phases = 1 is mr_conv2d_nhwc_tc. */
 int mr_conv2d_nhwc_tc_phases(const mr_conv_desc* descs, int n_phases, int n_pad, int k_pad, int round_out, void* stream);
+/* Launch plan of mr_conv2d_nhwc_tc_phases(descs, n_phases, n_pad, k_pad, round_out, ...) on a device with `sms` SMs (pure host
+ * code, callable without a GPU; the launch itself uses this function with the device's SM count).  Runs every argument check
+ * that needs no driver (MR_EINVAL and mr_last_error() like the launch) and reports which kernel, ring and epilogue the call
+ * takes.  The MONOREC_B200_TC_* switches above apply.
+ *   kernel       MR_TC_REFETCH: one input box and one weight slice per (tap, K chunk); strided layers, sub-pixel phases;
+ *                MR_TC_HALO: stride 1, one input box per (tile, K chunk), weights resident in shared memory;
+ *                MR_TC_HALO_STREAM: the same with the weights streamed through a ring of b_stream stages
+ *   ctas_per_sm  resident CTAs per SM the grid is sized for; stages: input ring stages (MR_TC_REFETCH: input + weight)
+ *   row_bytes    bytes of one K-chunk row in shared memory (128 or 64), kc: channels per K chunk
+ *   total_tiles  output tiles (8x16 pixels for MR_TC_REFETCH, 16x8 for the halo kernels) over batch and phases;
+ *                grid = min(sms * ctas_per_sm, total_tiles) persistent CTAs
+ *   epilogue     MR_TC_EPI_STAGED (LeakyReLU / no activation, 16-byte aligned channel slices), MR_TC_EPI_ONE_COLUMN (Cout == 1),
+ *                MR_TC_EPI_GENERIC (everything else) */
+#define MR_TC_REFETCH 0
+#define MR_TC_HALO 1
+#define MR_TC_HALO_STREAM 2
+#define MR_TC_EPI_STAGED 0
+#define MR_TC_EPI_ONE_COLUMN 1
+#define MR_TC_EPI_GENERIC 2
+typedef struct mr_conv_tc_plan {
+    int kernel, ctas_per_sm, stages, b_stream, row_bytes, kc;
+    int tmem_cols;                           /* tensor-memory columns per CTA (two accumulators) */
+    int smem_bytes;                          /* dynamic shared memory per CTA */
+    int total_tiles, grid, epilogue;
+} mr_conv_tc_plan;
+int mr_conv2d_nhwc_tc_plan(const mr_conv_desc* descs, int n_phases, int n_pad, int k_pad, int round_out, int sms,
+                           mr_conv_tc_plan* out);
 /* Host-side weight packing for mr_conv2d_nhwc_tc (pure host code, callable without a GPU).
  *   mr_pack_conv_weights_bytes: size of the packed tensor and its n_pad / k_pad for a correlation kernel (Cout, sum src_c, kh, kw)
  *     whose input channels are the concatenation of n_src sources; dtype MR_DT_F32 (TF32-rounded fp32) or MR_DT_F16.

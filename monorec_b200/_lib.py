@@ -40,6 +40,7 @@ SIGNATURES = {
     "mr_conv_workspace_bytes": (c_longlong, [c_void_p]),
     "mr_conv2d_nhwc_tc": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p]),
     "mr_conv2d_nhwc_tc_phases": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
+    "mr_conv2d_nhwc_tc_plan": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p]),
     "mr_nchw_to_nhwc": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),
     "mr_nchw_to_nhwc_f16": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),
     "mr_maxpool2_nhwc_f16": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p]),

@@ -340,24 +340,43 @@ class PackedConv:
                       act_b=self.act_b, out=out, pad=self.pad, out_hw=out_hw, out_step=self.out_step, out_off=self.out_off)
 
 
+def _tc_out(srcs, L, out, out_hw, half, out_f32):
+    """(destination, output grid) of a PackedConv on the tensor cores: `out` or a new NHWC tensor."""
+    x0 = srcs[0]
+    B, Hs, Ws, _ = x0.shape
+    if out_hw is None:
+        out_hw = (math.ceil(Hs / L.stride[0]), math.ceil(Ws / L.stride[1]))
+    if out is None:
+        out = torch.empty(B, out_hw[0] * L.out_step[0], out_hw[1] * L.out_step[1], L.cout, device=x0.device,
+                          dtype=torch.float16 if (half and not out_f32) else torch.float32)
+    return out, out_hw
+
+
+def _tc_descs(srcs, subs, out, out_hw, half, out_coff=0):
+    """Descriptors of one tensor-core launch over the PackedConvs `subs` (one, or the sub-pixel phases of a layer, which share
+    the first one's bias), with their packed weights' n_pad / k_pad."""
+    descs = (ConvDesc * len(subs))()
+    n_pad = k_pad = None
+    for d, L in zip(descs, subs):
+        wtc, n_pad_i, k_pad_i = L.wtc(half)
+        assert n_pad in (None, n_pad_i) and k_pad in (None, k_pad_i)
+        n_pad, k_pad = n_pad_i, k_pad_i
+        Hs, Ws = srcs[0].shape[1:3]
+        pad = L.pad if L.pad is not None else (same_pad_before(Hs, L.kh, L.stride[0]), same_pad_before(Ws, L.kw, L.stride[1]))
+        _fill_desc(d, srcs, L, out, out_hw, pad, wtc, half, out_coff)
+        d.bias = subs[0].bias.data_ptr() if subs[0].bias is not None else None
+    return descs, n_pad, k_pad
+
+
 def conv2d_tc(srcs, L, out=None, out_hw=None, round_out=True, half=False, out_f32=False, out_coff=0):
     """Tensor-core launch (csrc/conv_tc.cu) of a PackedConv."""
     lib = _lib.load()
     x0 = srcs[0]
-    B, Hs, Ws, _ = x0.shape
-    sy, sx = L.stride
-    pad = L.pad if L.pad is not None else (same_pad_before(Hs, L.kh, sy), same_pad_before(Ws, L.kw, sx))
-    if out_hw is None:
-        out_hw = (math.ceil(Hs / sy), math.ceil(Ws / sx))
-    Ho, Wo = out_hw
-    if out is None:
-        out = torch.empty(B, Ho * L.out_step[0], Wo * L.out_step[1], L.cout, device=x0.device,
-                          dtype=torch.float16 if (half and not out_f32) else torch.float32)
-    wtc, n_pad, k_pad = L.wtc(half)
-    d = ConvDesc()
-    _fill_desc(d, srcs, L, out, (Ho, Wo), pad, wtc, half, out_coff)
+    assert all(s.is_cuda for s in srcs)
+    out, out_hw = _tc_out(srcs, L, out, out_hw, half, out_f32)
+    descs, n_pad, k_pad = _tc_descs(srcs, [L], out, out_hw, half, out_coff)
     with torch.cuda.device(x0.device):
-        _lib.check(lib.mr_conv2d_nhwc_tc(ctypes.byref(d), n_pad, k_pad, int(round_out), _stream(x0)), "mr_conv2d_nhwc_tc")
+        _lib.check(lib.mr_conv2d_nhwc_tc(descs, n_pad, k_pad, int(round_out), _stream(x0)), "mr_conv2d_nhwc_tc")
     return out
 
 
@@ -368,7 +387,7 @@ def _fill_desc(d, srcs, L, out, out_hw, pad, wtc, half, out_coff=0):
     Ho, Wo = out_hw
     d.n_src = len(srcs)
     for i, s in enumerate(srcs):
-        assert s.is_cuda and s.dtype == (torch.float16 if half else torch.float32) and s.is_contiguous()
+        assert s.dtype == (torch.float16 if half else torch.float32) and s.is_contiguous()
         assert s.shape[:3] == x0.shape[:3]
         d.src[i] = s.data_ptr()
         d.src_c[i] = s.shape[3]
@@ -390,19 +409,46 @@ def conv2d_tc_phases(srcs, subs, out, out_hw, round_out=True, half=False):
     read from HBM once instead of once per phase."""
     lib = _lib.load()
     x0 = srcs[0]
-    descs = (ConvDesc * len(subs))()
-    n_pad = k_pad = None
-    keep = []
-    for d, L in zip(descs, subs):
-        wtc, n_pad_i, k_pad_i = L.wtc(half)
-        assert n_pad in (None, n_pad_i) and k_pad in (None, k_pad_i)
-        n_pad, k_pad = n_pad_i, k_pad_i
-        keep.append(wtc)
-        _fill_desc(d, srcs, L, out, out_hw, L.pad, wtc, half)
-        d.bias = subs[0].bias.data_ptr() if subs[0].bias is not None else None     # (one bias vector for all phases)
+    assert all(s.is_cuda for s in srcs) and all(L.pad is not None for L in subs)
+    descs, n_pad, k_pad = _tc_descs(srcs, subs, out, out_hw, half)
     with torch.cuda.device(x0.device):
         _lib.check(lib.mr_conv2d_nhwc_tc_phases(descs, len(subs), n_pad, k_pad, int(round_out), _stream(x0)), "mr_conv2d_nhwc_tc_phases")
     return out
+
+
+class TcPlan(ctypes.Structure):
+    """Mirror of `struct mr_conv_tc_plan` (include/monorec_b200.h)."""
+    _fields_ = [(n, c_int) for n in ("kernel", "ctas_per_sm", "stages", "b_stream", "row_bytes", "kc", "tmem_cols", "smem_bytes",
+                                     "total_tiles", "grid", "epilogue")]
+
+
+TC_KERNELS = ("refetch", "halo", "halo_stream")          # MR_TC_REFETCH, MR_TC_HALO, MR_TC_HALO_STREAM
+TC_EPILOGUES = ("staged", "one_column", "generic")       # MR_TC_EPI_*
+
+
+def tc_plan(layer, srcs, out=None, out_hw=None, round_out=True, half=False, out_f32=False, out_coff=0, sms=None):
+    """Launch plan (mr_conv2d_nhwc_tc_plan) of `conv2d_tc(srcs, layer, out, out_hw, round_out, half, out_f32, out_coff)` for a
+    PackedConv, or of the one-launch call a PackedSubpixel makes (`out`: its (2H, 2W) destination), as a dict.  Host code only:
+    the sources may be CPU tensors.  sms: SM count the grid is sized for (default: that of the sources' device)."""
+    lib = _lib.load()
+    x0 = srcs[0]
+    if isinstance(layer, PackedSubpixel):
+        subs = layer.subs
+        if out is None:
+            out = torch.empty(x0.shape[0], 2 * x0.shape[1], 2 * x0.shape[2], subs[0].cout, device=x0.device, dtype=x0.dtype)
+        out_hw = tuple(x0.shape[1:3])
+    else:
+        subs = [layer]
+        out, out_hw = _tc_out(srcs, layer, out, out_hw, half, out_f32)
+    if sms is None:
+        sms = torch.cuda.get_device_properties(x0.device).multi_processor_count
+    descs, n_pad, k_pad = _tc_descs(srcs, subs, out, out_hw, half, out_coff)
+    p = TcPlan()
+    _lib.check(lib.mr_conv2d_nhwc_tc_plan(descs, len(subs), n_pad, k_pad, int(round_out), int(sms), ctypes.byref(p)),
+               "mr_conv2d_nhwc_tc_plan")
+    r = {n: getattr(p, n) for n, _ in TcPlan._fields_}
+    r["kernel"], r["epilogue"], r["n_phases"] = TC_KERNELS[p.kernel], TC_EPILOGUES[p.epilogue], len(subs)
+    return r
 
 
 # MONOREC_B200_SUBPIXEL_ONE_LAUNCH=0: one launch per sub-pixel phase (A/B measurements)

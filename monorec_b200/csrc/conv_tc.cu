@@ -65,6 +65,7 @@ struct TcArgs {
                                    // [n_pad x chunk] slice of every (chunk, tap) streams through a ring of n stages instead
     int halo_pitch;                // halo kernel: pixels per input row of the shared-memory box (8 outputs + kw - 1 taps to the right)
     uint32_t halo_a_bytes;         // halo kernel: bytes of one input stage (box rounded up to 1 KB)
+    int epi;                       // MR_TC_EPI_*: the epilogue the host plan chose
 };
 
 // ---- PTX wrappers -------------------------------------------------------------------------------------------------------
@@ -187,6 +188,13 @@ __device__ __forceinline__ float act_fn(float v, int act, float a, float b) {
     }
 }
 
+// LeakyReLU x >= 0 ? x : s*x for any slope as one min / max: max(x, s*x) when s <= 1, min(x, s*x) when s > 1.  `s_le1` is the
+// same for the whole layer, so the choice costs no per-element predicate (FMNMX takes it as an operand).
+__device__ __forceinline__ float leaky(float x, float s, bool s_le1) {
+    const float y = s * x;
+    return s_le1 ? fmaxf(x, y) : fminf(x, y);
+}
+
 // Epilogue of one accumulator row (= one output pixel): 32 columns per step (two x16 TMEM loads, one wait), bias from shared
 // memory, activation, optional TF32 rounding, 16-byte NHWC stores.
 __device__ __forceinline__ void epilogue_row(uint32_t trow, const TcArgs& a, const float* bias_s, float* op, bool live,
@@ -207,8 +215,7 @@ __device__ __forceinline__ void epilogue_row(uint32_t trow, const TcArgs& a, con
 #pragma unroll
             for (int j = 0; j < 16; ++j) {
                 float x = __uint_as_float(h ? r1[j] : r0[j]) + bias_s[nb + j];
-                if (a.act == MR_ACT_LEAKY) x = fmaxf(x, a.act_a * x);          // slope in (0, 1)
-                else if (a.act != MR_ACT_NONE) x = act_fn(x, a.act, a.act_a, a.act_b);
+                if (a.act != MR_ACT_NONE) x = act_fn(x, a.act, a.act_a, a.act_b);
                 if (a.round_out) x = __uint_as_float((__float_as_uint(x) + 0x1000u) & 0xFFFFE000u);
                 v[j] = x;
             }
@@ -248,7 +255,7 @@ __device__ __noinline__ void epilogue_row_outofline(uint32_t trow, const TcArgs 
 // The source-level profile of round 1's register epilogue (profiles/r01_k2_fullres_f16_quad_ncu_details.txt and the source page of
 // the same capture) shows ~900 executed instructions per warp and tile spread over a 12 700-instruction kernel body
 // (23 % of the stall samples are instruction-fetch misses) -- per-element activation switches, predicates and 48 SEL + 16
-// SHFL per quad transpose.  This variant keeps the per-tile decisions out of the element loop (LeakyReLU as max(x, slope*x)
+// SHFL per quad transpose.  This variant keeps the per-tile decisions out of the element loop (LeakyReLU through leaky()
 // with slope = 1 for "no activation", rounding as a template parameter) and transposes through a 2 KB per-warp staging
 // buffer in shared memory instead of shuffles: every thread writes the 64 bytes of its pixel (4 x STS.128, XOR-swizzled,
 // conflict-free), then lane l reads chunk l%4 of pixel l/4 + 8k and stores it, so that one store instruction covers 8
@@ -258,6 +265,7 @@ __device__ __forceinline__ void epilogue_staged(uint32_t trow, const TcArgs& a, 
                                                 const bool (&qlive)[4], int lane, float slope) {
     constexpr int kCols = OUT_F16 ? 32 : 16;        // output channels per 64-byte step
     constexpr int kChunk = OUT_F16 ? 8 : 4;         // channels per 16-byte chunk
+    const bool s_le1 = slope <= 1.f;
     const uint32_t wrow = stg + (uint32_t)lane * 64u;
     const uint32_t wsw = ((uint32_t)lane >> 1) & 3u;
     const uint32_t c = (uint32_t)lane & 3u;
@@ -279,13 +287,13 @@ __device__ __forceinline__ void epilogue_staged(uint32_t trow, const TcArgs& a, 
 #pragma unroll
             for (int j = 0; j < 8; ++j) {
                 float x0 = __uint_as_float(r0[2 * j]) + bias_s[n0 + 2 * j], x1 = __uint_as_float(r0[2 * j + 1]) + bias_s[n0 + 2 * j + 1];
-                h[j] = __floats2half2_rn(fmaxf(x0, slope * x0), fmaxf(x1, slope * x1));
+                h[j] = __floats2half2_rn(leaky(x0, slope, s_le1), leaky(x1, slope, s_le1));
             }
             if (second) {
 #pragma unroll
                 for (int j = 0; j < 8; ++j) {
                     float x0 = __uint_as_float(r1[2 * j]) + bias_s[n0 + 16 + 2 * j], x1 = __uint_as_float(r1[2 * j + 1]) + bias_s[n0 + 17 + 2 * j];
-                    h[8 + j] = __floats2half2_rn(fmaxf(x0, slope * x0), fmaxf(x1, slope * x1));
+                    h[8 + j] = __floats2half2_rn(leaky(x0, slope, s_le1), leaky(x1, slope, s_le1));
                 }
             } else {
                 e[2] = make_uint4(0u, 0u, 0u, 0u);
@@ -296,7 +304,7 @@ __device__ __forceinline__ void epilogue_staged(uint32_t trow, const TcArgs& a, 
 #pragma unroll
             for (int j = 0; j < 16; ++j) {
                 float x = __uint_as_float(r0[j]) + bias_s[n0 + j];
-                x = fmaxf(x, slope * x);
+                x = leaky(x, slope, s_le1);
                 w[j] = ROUND ? ((__float_as_uint(x) + 0x1000u) & 0xFFFFE000u) : __float_as_uint(x);
             }
         }
@@ -346,7 +354,7 @@ __device__ __forceinline__ void staged_tile(const TcArgs& a, const float* bias_s
         const size_t oidx = (((size_t)b * a.dst_H + (oy * a.oy_step + oy_off)) * a.dst_W + (ox * a.ox_step + ox_off)) *
                                 a.dst_c + a.dst_coff;
         const bool live = (oy < a.Ho) && (ox < a.Wo);
-        if (a.Cout == 1) {
+        if (a.epi == MR_TC_EPI_ONE_COLUMN) {
             // single-channel heads (sigmoid / a + b |tanh|): one accumulator column per pixel instead of the generic path's 16
             // activations per pixel (measured: 24->1 3x3 at full resolution 123 us with the generic epilogue)
             uint32_t r;
@@ -488,8 +496,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
         const int q = warp & 3;                 // TMEM lane quadrant this warp may read (the 4 epilogue warps have distinct ones)
         const uint32_t stg = smem_u32(&stage_s[q][0]);
         const bool vec_ok = ((a.dst_c | a.dst_coff) & (a.out_f16 ? 7 : 3)) == 0;
-        const bool lean_ok = vec_ok && (a.Cout & (a.out_f16 ? 7 : 3)) == 0 && !(a.out_f16 && a.round_out) &&
-                             (a.act == MR_ACT_NONE || a.act == MR_ACT_LEAKY);
+        const bool lean_ok = a.epi == MR_TC_EPI_STAGED;
         const float slope = a.act == MR_ACT_LEAKY ? a.act_a : 1.0f;
         int lt = 0;
         for (int tile = blockIdx.x; tile < a.total_tiles; tile += gridDim.x, ++lt) {
@@ -675,8 +682,7 @@ conv_tc_halo_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_const
         const int q = warp & 3;                 // TMEM lane quadrant
         const uint32_t stg = smem_u32(&stage_s[warp - 2][0]);
         const bool vec_ok = ((a.dst_c | a.dst_coff) & (a.out_f16 ? 7 : 3)) == 0;
-        const bool lean_ok = vec_ok && (a.Cout & (a.out_f16 ? 7 : 3)) == 0 && !(a.out_f16 && a.round_out) &&
-                             (a.act == MR_ACT_NONE || a.act == MR_ACT_LEAKY);
+        const bool lean_ok = a.epi == MR_TC_EPI_STAGED;
         const float slope = a.act == MR_ACT_LEAKY ? a.act_a : 1.0f;
         int lt = 0;
         for (int tile = blockIdx.x; tile < a.total_tiles; tile += gridDim.x, ++lt) {
@@ -719,9 +725,13 @@ EncodeTiledFn get_encode_fn() {
 
 }  // namespace
 
-static int conv2d_nhwc_tc_impl(const mr_conv_desc* desc, int n_phases, int n_pad, int k_pad, int round_out, void* stream) {
+// The launch plan: argument checks, kernel choice, ring depths, grid and epilogue of one call, on the host without the driver.
+// `a` receives the kernel arguments (everything but the tensor maps, which need the driver).
+static int conv2d_nhwc_tc_plan_impl(const mr_conv_desc* desc, int n_phases, int n_pad, int k_pad, int round_out, int sms,
+                                    mr_conv_tc_plan* plan, TcArgs& a) {
     MR_REQUIRE(desc != nullptr, "mr_conv2d_nhwc_tc: null descriptor");
     MR_REQUIRE(n_phases >= 1 && n_phases <= 4, "mr_conv2d_nhwc_tc_phases: 1..4 phases (got %d)", n_phases);
+    MR_REQUIRE(sms >= 1, "mr_conv2d_nhwc_tc_plan: sms=%d", sms);
     const mr_conv_desc& d = desc[0];
     for (int p = 1; p < n_phases; ++p) {   // phases share everything but the filter (size, padding, weights) and the output offset
         const mr_conv_desc& e = desc[p];
@@ -730,7 +740,7 @@ static int conv2d_nhwc_tc_impl(const mr_conv_desc* desc, int n_phases, int n_pad
                     e.dst_H == d.dst_H && e.dst_W == d.dst_W && e.dst_c == d.dst_c && e.dst_coff == d.dst_coff &&
                     e.oy_step == d.oy_step && e.ox_step == d.ox_step && e.act == d.act && e.act_a == d.act_a && e.act_b == d.act_b &&
                     e.src_dtype == d.src_dtype && e.dst_dtype == d.dst_dtype;
-        for (int s = 0; same && s < d.n_src; ++s) same = e.src[s] == d.src[s] && e.src_c[s] == d.src_c[s];
+        for (int s = 0; same && s < d.n_src && s < MR_CONV_MAX_SRC; ++s) same = e.src[s] == d.src[s] && e.src_c[s] == d.src_c[s];
         MR_REQUIRE(same, "mr_conv2d_nhwc_tc_phases: phase %d differs from phase 0 in more than filter size, padding, weights and output offset", p);
         MR_REQUIRE(e.weight && e.kh >= 1 && e.kw >= 1 && (e.Ho - 1) * e.oy_step + e.oy_off < e.dst_H && (e.Wo - 1) * e.ox_step + e.ox_off < e.dst_W,
                    "mr_conv2d_nhwc_tc_phases: phase %d: bad filter / output placement", p);
@@ -746,15 +756,10 @@ static int conv2d_nhwc_tc_impl(const mr_conv_desc* desc, int n_phases, int n_pad
     MR_REQUIRE(d.dst_coff >= 0 && d.dst_coff + d.Cout <= d.dst_c, "mr_conv2d_nhwc_tc: channel slice out of range");
     MR_REQUIRE((d.Ho - 1) * d.oy_step + d.oy_off < d.dst_H && (d.Wo - 1) * d.ox_step + d.ox_off < d.dst_W,
                "mr_conv2d_nhwc_tc: output placement out of range");
-    EncodeTiledFn encode = get_encode_fn();
-    if (encode == nullptr) {
-        mr::set_error("mr_conv2d_nhwc_tc: cuTensorMapEncodeTiled is not available from this driver");
-        return MR_ENOSUPPORT;
-    }
-    TcArgs a{};
-    a.n_src = d.n_src;
+    MR_REQUIRE(d.act >= MR_ACT_NONE && d.act <= MR_ACT_ABSTANH, "mr_conv2d_nhwc_tc: unknown activation %d", d.act);
     MR_REQUIRE(d.src_dtype == MR_DT_F32 || d.src_dtype == MR_DT_F16, "mr_conv2d_nhwc_tc: bad src_dtype %d", d.src_dtype);
     MR_REQUIRE(d.dst_dtype == MR_DT_F32 || d.dst_dtype == MR_DT_F16, "mr_conv2d_nhwc_tc: bad dst_dtype %d", d.dst_dtype);
+    a.n_src = d.n_src;
     const bool f16 = d.src_dtype == MR_DT_F16;
     // K chunk = one swizzle row of channels: 32 fp32 or 64 half (128 bytes).  Half sources whose channel counts waste less
     // with 32-channel chunks (32, 96, ... channels) are packed that way by the caller (k_pad tells): 64-byte rows, SWIZZLE_64B,
@@ -773,6 +778,17 @@ static int conv2d_nhwc_tc_impl(const mr_conv_desc* desc, int n_phases, int n_pad
     // F16 = 0; K-major A and B; N >> 3 @[17,23); M >> 4 @[24,29)
     a.idesc = (1u << 4) | ((f16 ? 0u : 2u) << 7) | ((f16 ? 0u : 2u) << 10) | ((uint32_t)(n_pad >> 3) << 17) | ((128u >> 4) << 24);
     int ksum = 0;
+    for (int s = 0; s < d.n_src; ++s) {
+        const int C = d.src_c[s];
+        MR_REQUIRE(d.src[s] != nullptr && C >= cmult && (C % cmult) == 0,
+                   "mr_conv2d_nhwc_tc: source %d needs a channel count that is a multiple of %d (got %d)", s, cmult, C);
+        MR_REQUIRE((reinterpret_cast<uintptr_t>(d.src[s]) & 15) == 0, "mr_conv2d_nhwc_tc: source %d is not 16-byte aligned", s);
+        a.chunks[s] = (C + kc - 1) / kc;
+        a.tail_ksteps[s] = ((C - (a.chunks[s] - 1) * kc) * esize + 31) / 32;
+        ksum += a.chunks[s] * kc;
+    }
+    MR_REQUIRE(ksum == k_pad, "mr_conv2d_nhwc_tc: packed weight K (%d) does not match the sources (%d)", k_pad, ksum);
+    MR_REQUIRE((reinterpret_cast<uintptr_t>(d.weight) & 15) == 0, "mr_conv2d_nhwc_tc: weights are not 16-byte aligned");
     // "halo" variant (one input box per tile, resident weights): stride 1, taps reach at most 8 px to the right, weights fit
     int chunks_all = 0;
     for (int s = 0; s < d.n_src; ++s) chunks_all += (d.src_c[s] + kc - 1) / kc;
@@ -829,51 +845,6 @@ static int conv2d_nhwc_tc_impl(const mr_conv_desc* desc, int n_phases, int n_pad
         }
     }
     const bool halo = halo_ctas > 0;
-    const int halo_stages = b_stream ? stream_stages : (halo ? halo_fit(halo_ctas) : 0);
-    const size_t halo_front = b_stream ? (size_t)b_stream * b_slice : bres_al;   // bytes in front of the input stages
-    CUtensorMap tmA[MR_CONV_MAX_SRC];
-    for (int s = 0; s < d.n_src; ++s) {
-        const int C = d.src_c[s];
-        MR_REQUIRE(d.src[s] != nullptr && C >= cmult && (C % cmult) == 0,
-                   "mr_conv2d_nhwc_tc: source %d needs a channel count that is a multiple of %d (got %d)", s, cmult, C);
-        MR_REQUIRE((reinterpret_cast<uintptr_t>(d.src[s]) & 15) == 0, "mr_conv2d_nhwc_tc: source %d is not 16-byte aligned", s);
-        a.chunks[s] = (C + kc - 1) / kc;
-        a.tail_ksteps[s] = ((C - (a.chunks[s] - 1) * kc) * esize + 31) / 32;
-        ksum += a.chunks[s] * kc;
-        const cuuint64_t gdim[4] = {(cuuint64_t)C, (cuuint64_t)d.Ws, (cuuint64_t)d.Hs, (cuuint64_t)d.B};
-        const cuuint64_t gstr[3] = {(cuuint64_t)C * esize, (cuuint64_t)d.Ws * C * esize, (cuuint64_t)d.Hs * d.Ws * C * esize};
-        // with a traversal stride s the box spans box/s loaded elements: 16 (8) output pixels need a span of 16*s (8*s)
-        cuuint32_t box[4] = {(cuuint32_t)kc, (cuuint32_t)(kTileW * d.sx), (cuuint32_t)(kTileH * d.sy), 1};
-        if (halo) { box[1] = (cuuint32_t)halo_pitch; box[2] = (cuuint32_t)(16 + d.kh - 1); }
-        const cuuint32_t estr[4] = {1, (cuuint32_t)d.sx, (cuuint32_t)d.sy, 1};
-        CUresult r = encode(&tmA[s], f16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<float*>(d.src[s]), gdim, gstr, box, estr,
-                            CU_TENSOR_MAP_INTERLEAVE_NONE, a.row_bytes == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B,
-                            CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) {
-            mr::set_error("mr_conv2d_nhwc_tc: cuTensorMapEncodeTiled(A%d) failed with CUresult %d", s, (int)r);
-            return MR_EINVAL;
-        }
-    }
-    for (int s = d.n_src; s < MR_CONV_MAX_SRC; ++s) tmA[s] = tmA[0];
-    MR_REQUIRE(ksum == k_pad, "mr_conv2d_nhwc_tc: packed weight K (%d) does not match the sources (%d)", k_pad, ksum);
-    MR_REQUIRE((reinterpret_cast<uintptr_t>(d.weight) & 15) == 0, "mr_conv2d_nhwc_tc: weights are not 16-byte aligned");
-    CUtensorMap tmBs[4];
-    for (int p = 0; p < n_phases; ++p) {
-        const mr_conv_desc& e = desc[p];
-        const cuuint64_t gdim[2] = {(cuuint64_t)k_pad, (cuuint64_t)e.kh * e.kw * n_pad};
-        const cuuint64_t gstr[1] = {(cuuint64_t)k_pad * esize};
-        const cuuint32_t box[2] = {(cuuint32_t)kc, (cuuint32_t)n_pad};
-        const cuuint32_t estr[2] = {1, 1};
-        CUresult r = encode(&tmBs[p], f16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float*>(e.weight), gdim, gstr, box, estr,
-                            CU_TENSOR_MAP_INTERLEAVE_NONE, a.row_bytes == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B,
-                            CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) {
-            mr::set_error("mr_conv2d_nhwc_tc: cuTensorMapEncodeTiled(B) failed with CUresult %d", (int)r);
-            return MR_EINVAL;
-        }
-    }
-    for (int p = n_phases; p < 4; ++p) tmBs[p] = tmBs[0];
-    const CUtensorMap& tmB = tmBs[0];
     a.n_phase = n_phases;
     for (int p = 0; p < 4; ++p) {
         const mr_conv_desc& e = desc[p < n_phases ? p : 0];
@@ -883,57 +854,131 @@ static int conv2d_nhwc_tc_impl(const mr_conv_desc* desc, int n_phases, int n_pad
     a.Ho = d.Ho; a.Wo = d.Wo; a.Cout = d.Cout; a.n_pad = n_pad;
     a.tiles_x = halo ? (d.Wo + 7) / 8 : (d.Wo + kTileW - 1) / kTileW;
     const int tiles = a.tiles_x * (halo ? (d.Ho + 15) / 16 : (d.Ho + kTileH - 1) / kTileH);
-    const size_t stage_bytes = (size_t)(128 + n_pad) * a.row_bytes;
     a.tiles_per_img = tiles;
     a.total_tiles = tiles * d.B * n_phases;
-    // persistent grid: two CTAs per SM when two double-buffered accumulators fit TMEM (2 x 2 x n_pad <= 512 columns),
-    // otherwise one CTA per SM with a deeper ring
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    // tap-refetch kernel, persistent grid: resident CTAs per SM bounded by TMEM (each CTA holds a power-of-two >= 2 * n_pad columns
+    // of the 512) and capped at 4; with UMMA N = 32..64 one CTA cannot keep the tensor pipe busy, so several CTAs interleave
+    // their MMA chains; the ring takes what shared memory is left
     static const int kForceCtas = getenv("MONOREC_B200_TC_CTAS") ? atoi(getenv("MONOREC_B200_TC_CTAS")) : 0;   // tuning knob
-    // resident CTAs per SM: bounded by TMEM (each CTA holds a power-of-two >= 2 * n_pad columns of the 512) and capped at 4;
-    // with UMMA N = 32..64 one CTA cannot keep the tensor pipe busy, so several CTAs interleave their MMA chains
-    uint32_t cols_needed = 32;
-    while (cols_needed < (uint32_t)(2 * n_pad)) cols_needed <<= 1;
-    int ctas_per_sm = (int)(512 / cols_needed);
-    if (ctas_per_sm > 4) ctas_per_sm = 4;
-    if (kForceCtas > 0 && (uint32_t)kForceCtas * cols_needed <= 512) ctas_per_sm = kForceCtas;
-    const size_t budget = (size_t)(200 * 1024) / ctas_per_sm - 8 * 1024;
-    int stages = (int)(budget / stage_bytes);
-    if (stages > 8) stages = 8;
-    if (stages < 2) stages = 2;
-    a.stages = stages;
     uint32_t cols = 32;
     while (cols < (uint32_t)(2 * n_pad)) cols <<= 1;
     a.tmem_cols = cols;
+    int ctas_per_sm = (int)(512 / cols);
+    if (ctas_per_sm > 4) ctas_per_sm = 4;
+    if (kForceCtas > 0 && (uint32_t)kForceCtas * cols <= 512) ctas_per_sm = kForceCtas;
+    const size_t stage_bytes = (size_t)(128 + n_pad) * a.row_bytes;
+    int stages = (int)(((size_t)(200 * 1024) / ctas_per_sm - 8 * 1024) / stage_bytes);
+    if (stages > 8) stages = 8;
+    if (stages < 2) stages = 2;
+    size_t smem = (size_t)stages * stage_bytes + 1024;
+    if (halo) {
+        ctas_per_sm = halo_ctas;
+        stages = b_stream ? stream_stages : halo_fit(halo_ctas);
+        const size_t halo_front = b_stream ? (size_t)b_stream * b_slice : bres_al;   // bytes in front of the input stages
+        smem = halo_front + (size_t)stages * halo_a_bytes + 1024;
+        a.halo_pitch = halo_pitch;
+        a.halo_a_bytes = (uint32_t)halo_a_bytes;
+        a.b_stream = b_stream;
+    }
+    a.stages = stages;
     a.bias = d.bias; a.dst = d.dst;
     a.dst_H = d.dst_H; a.dst_W = d.dst_W; a.dst_c = d.dst_c; a.dst_coff = d.dst_coff;
     a.oy_step = d.oy_step; a.ox_step = d.ox_step; a.oy_off = d.oy_off; a.ox_off = d.ox_off;
     a.act = d.act; a.act_a = d.act_a; a.act_b = d.act_b; a.round_out = round_out;
+    // staged epilogue: 16-byte stores of whole channel groups, no activation or LeakyReLU; one-channel heads take one accumulator
+    // column; anything else (unaligned channel slices, Cout not a multiple of 4 / 8, sigmoid / |tanh| with Cout > 1) is generic
+    const int vmask = a.out_f16 ? 7 : 3;
+    if (((d.dst_c | d.dst_coff | d.Cout) & vmask) == 0 && !(a.out_f16 && round_out) && (d.act == MR_ACT_NONE || d.act == MR_ACT_LEAKY))
+        a.epi = MR_TC_EPI_STAGED;
+    else
+        a.epi = d.Cout == 1 ? MR_TC_EPI_ONE_COLUMN : MR_TC_EPI_GENERIC;
+    int grid = sms * ctas_per_sm;
+    if (grid > a.total_tiles) grid = a.total_tiles;
+    plan->kernel = !halo ? MR_TC_REFETCH : (b_stream ? MR_TC_HALO_STREAM : MR_TC_HALO);
+    plan->ctas_per_sm = ctas_per_sm;
+    plan->stages = stages;
+    plan->b_stream = b_stream;
+    plan->row_bytes = a.row_bytes;
+    plan->kc = kc;
+    plan->tmem_cols = (int)cols;
+    plan->smem_bytes = (int)smem;
+    plan->total_tiles = a.total_tiles;
+    plan->grid = grid;
+    plan->epilogue = a.epi;
+    return MR_OK;
+}
+
+extern "C" int mr_conv2d_nhwc_tc_plan(const mr_conv_desc* descs, int n_phases, int n_pad, int k_pad, int round_out, int sms,
+                                      mr_conv_tc_plan* out) {
+    MR_REQUIRE(out != nullptr, "mr_conv2d_nhwc_tc_plan: null plan");
+    TcArgs a{};
+    return conv2d_nhwc_tc_plan_impl(descs, n_phases, n_pad, k_pad, round_out, sms, out, a);
+}
+
+static int conv2d_nhwc_tc_impl(const mr_conv_desc* desc, int n_phases, int n_pad, int k_pad, int round_out, void* stream) {
+    int dev = 0, sms = 148;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    TcArgs a{};
+    mr_conv_tc_plan plan{};
+    const int prc = conv2d_nhwc_tc_plan_impl(desc, n_phases, n_pad, k_pad, round_out, sms, &plan, a);
+    if (prc != MR_OK) return prc;
+    EncodeTiledFn encode = get_encode_fn();
+    if (encode == nullptr) {
+        mr::set_error("mr_conv2d_nhwc_tc: cuTensorMapEncodeTiled is not available from this driver");
+        return MR_ENOSUPPORT;
+    }
+    const mr_conv_desc& d = desc[0];
+    const bool halo = plan.kernel != MR_TC_REFETCH;
+    const int esize = a.f16 ? 2 : 4;
+    const CUtensorMapDataType dtype = a.f16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
+    const CUtensorMapSwizzle swizzle = a.row_bytes == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B;
+    CUtensorMap tmA[MR_CONV_MAX_SRC];
+    for (int s = 0; s < d.n_src; ++s) {
+        const int C = d.src_c[s];
+        const cuuint64_t gdim[4] = {(cuuint64_t)C, (cuuint64_t)d.Ws, (cuuint64_t)d.Hs, (cuuint64_t)d.B};
+        const cuuint64_t gstr[3] = {(cuuint64_t)C * esize, (cuuint64_t)d.Ws * C * esize, (cuuint64_t)d.Hs * d.Ws * C * esize};
+        // with a traversal stride s the box spans box/s loaded elements: 16 (8) output pixels need a span of 16*s (8*s)
+        cuuint32_t box[4] = {(cuuint32_t)a.kc, (cuuint32_t)(kTileW * d.sx), (cuuint32_t)(kTileH * d.sy), 1};
+        if (halo) { box[1] = (cuuint32_t)a.halo_pitch; box[2] = (cuuint32_t)(16 + d.kh - 1); }
+        const cuuint32_t estr[4] = {1, (cuuint32_t)d.sx, (cuuint32_t)d.sy, 1};
+        CUresult r = encode(&tmA[s], dtype, 4, const_cast<float*>(d.src[s]), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                            swizzle, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+        if (r != CUDA_SUCCESS) {
+            mr::set_error("mr_conv2d_nhwc_tc: cuTensorMapEncodeTiled(A%d) failed with CUresult %d", s, (int)r);
+            return MR_EINVAL;
+        }
+    }
+    for (int s = d.n_src; s < MR_CONV_MAX_SRC; ++s) tmA[s] = tmA[0];
+    CUtensorMap tmBs[4];
+    for (int p = 0; p < n_phases; ++p) {
+        const mr_conv_desc& e = desc[p];
+        const cuuint64_t gdim[2] = {(cuuint64_t)k_pad, (cuuint64_t)e.kh * e.kw * n_pad};
+        const cuuint64_t gstr[1] = {(cuuint64_t)k_pad * esize};
+        const cuuint32_t box[2] = {(cuuint32_t)a.kc, (cuuint32_t)n_pad};
+        const cuuint32_t estr[2] = {1, 1};
+        CUresult r = encode(&tmBs[p], dtype, 2, const_cast<float*>(e.weight), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                            swizzle, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+        if (r != CUDA_SUCCESS) {
+            mr::set_error("mr_conv2d_nhwc_tc: cuTensorMapEncodeTiled(B) failed with CUresult %d", (int)r);
+            return MR_EINVAL;
+        }
+    }
+    for (int p = n_phases; p < 4; ++p) tmBs[p] = tmBs[0];
+    const size_t smem = (size_t)plan.smem_bytes;
     if (halo) {
-        a.stages = halo_stages;
-        a.halo_pitch = halo_pitch;
-        a.halo_a_bytes = (uint32_t)halo_a_bytes;
-        a.b_stream = b_stream;
-        const size_t smem = halo_front + (size_t)halo_stages * halo_a_bytes + 1024;
-        int grid = sms * halo_ctas;
-        if (grid > a.total_tiles) grid = a.total_tiles;
-        auto launch_halo = [&](auto kernel, int threads) -> int {
+        auto launch_halo = [&](auto kernel) -> int {
             MR_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(212 * 1024)));
-            kernel<<<grid, threads, smem, (cudaStream_t)stream>>>(tmA[0], tmA[1], tmA[2], tmB, a);
+            kernel<<<plan.grid, kTcThreads, smem, (cudaStream_t)stream>>>(tmA[0], tmA[1], tmA[2], tmBs[0], a);
             return MR_OK;
         };
-        const int lrc = a.row_bytes == 128 ? launch_halo(conv_tc_halo_kernel<128>, kTcThreads) : launch_halo(conv_tc_halo_kernel<64>, kTcThreads);
+        const int lrc = a.row_bytes == 128 ? launch_halo(conv_tc_halo_kernel<128>) : launch_halo(conv_tc_halo_kernel<64>);
         if (lrc != MR_OK) return lrc;
         MR_LAUNCH_CHECK("conv_tc_halo_kernel");
         return MR_OK;
     }
-    const size_t smem = (size_t)stages * stage_bytes + 1024;
-    int grid = sms * ctas_per_sm;
-    if (grid > a.total_tiles) grid = a.total_tiles;
     MR_CUDA(cudaFuncSetAttribute(conv_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(212 * 1024)));
-    conv_tc_kernel<<<grid, kTcThreads, smem, (cudaStream_t)stream>>>(tmA[0], tmA[1], tmA[2], tmBs[0], tmBs[1], tmBs[2], tmBs[3], a);
+    conv_tc_kernel<<<plan.grid, kTcThreads, smem, (cudaStream_t)stream>>>(tmA[0], tmA[1], tmA[2], tmBs[0], tmBs[1], tmBs[2], tmBs[3], a);
     MR_LAUNCH_CHECK("conv_tc_kernel");
     return MR_OK;
 }
